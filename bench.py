@@ -17,6 +17,10 @@ MeanConst(0) -- config C2 of SURVEY.md §8(d)).
   cpu_baseline the reference's algorithm (oracle port: scalar loops in C + LAPACK via OpenBLAS, all
                host cores) on a bounded sample (N=8192) of the same workload
   --impl reference   times only that CPU path (Julia is not installed in this image).
+  --dump-outputs DIR after the timed steps, writes what the last timed step of each GPU path returned to its caller
+                     as DIR/<name>.npy (float64): alpha, mll, dmll_kernel, trace_A (resident step), e2e_alpha, e2e_mll,
+                     e2e_dmll (e2e step), predict_mu, predict_var (predict_f).  Inputs are seeded, so two builds run
+                     with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -223,7 +227,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--n", type=int, default=N_FULL, help="override N (debug only; the metric is N=32768)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed steps as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -269,9 +276,10 @@ def main():
 
     def step_resident():
         eng.factorize(theta, LNOISE)
-        eng.mll(r)
+        alpha, mll = eng.mll(r)
         eng.grad_prepare()
-        return eng.grad_kernel()
+        gk, tr_a = eng.grad_kernel()
+        return {"alpha": alpha, "mll": mll, "dmll_kernel": gk, "trace_A": tr_a}
 
     def step_e2e():
         gp.reload_data(Xh.T, yh)            # H2D of x and (inside update_mll) y
@@ -292,7 +300,7 @@ def main():
     sampler.start()
     e0.record(stream)
     for _ in range(args.steps):
-        step_resident()
+        outputs = step_resident()
     e1.record(stream)
     barrier()
     clocks = sampler.stop()
@@ -318,6 +326,7 @@ def main():
     e1.record(stream)
     barrier()
     e2e_wall = (time.perf_counter() - t0) * 1e3 / args.steps
+    outputs.update(e2e_alpha=gp.alpha.copy(), e2e_mll=gp.mll, e2e_dmll=gp.dmll.copy())
     e2e_ms = max(e0.elapsed_time(e1) / args.steps, e2e_wall)
     if world > 1:
         t = torch.tensor([e2e_ms], dtype=torch.float64, device="cuda")
@@ -364,6 +373,7 @@ def main():
         mu_p, var_p, _ = eng.predict(Xs)
         pms.append(eng.timings()["predict"])
     predict_ms = float(np.median(pms))
+    outputs.update(predict_mu=mu_p, predict_var=var_p)
     check["predict_mu_l1"] = float(np.sum(np.abs(mu_p)))
     check["predict_var_sum"] = float(np.sum(var_p))
     hbm_peak = None
@@ -426,6 +436,10 @@ def main():
             "check": check,
             "cpu_baseline": cpu,
         }
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, v in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), np.atleast_1d(np.asarray(v, dtype=np.float64)))
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,17 +1,18 @@
-"""Build tests/golden/simdata_kat.npz from the reference tree (run in the build container only).
+"""Build tests/golden/simdata_kat.npz from a checkout of GaussianProcesses.jl:
 
-Source of the known-answer vector (paths relative to /root/reference):
+    python tests/golden/make_golden.py <path to GaussianProcesses.jl>
+
+Source of the known-answer vector (paths relative to that checkout):
   perf/benchmarks/simdata.csv                              3000 x 10 inputs + Y
   perf/benchmarks/notebooks/benchmark_julia.ipynb cell 6   recorded output of the reference:
       GPE(X, Y, MeanConst(0.0), SEIso(0.0,0.0), log(1.0))  ->  mll, dmll
 The recorded run used the 2018 package version that added a 1e-5 diagonal jitter; the current
 source (src/GPE.jl:173-174) has none.  Both are pinned in tests/test_oracle_golden.py.
-/root/reference does not exist on the GPU box, hence the committed .npz.
+The tests do not need that checkout: they read the committed .npz.
 """
 import json, os, sys
 import numpy as np
 
-REF = "/root/reference"
 here = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -30,6 +31,7 @@ def recorded_from_notebook():
 
 
 if __name__ == "__main__":
+    REF = sys.argv[1]
     raw = np.loadtxt(os.path.join(REF, "perf/benchmarks/simdata.csv"), delimiter=",", skiprows=1)
     assert raw.shape == (3000, 11)
     txt = recorded_from_notebook()

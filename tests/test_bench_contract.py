@@ -57,6 +57,38 @@ def test_reference_arm_other_ranks_stay_silent():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+@pytest.mark.gpu
+def test_dump_outputs_hold_what_the_timed_steps_returned(tmp_path):
+    """--dump-outputs writes float64 arrays of the last timed steps; on bench.py's own seeded inputs they equal the oracle
+    (tolerances of the parity tests)."""
+    import bench
+    from oracle import gp_oracle as orc
+    n = 1536
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--n", str(n), "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    j = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+    assert j["steps"] == 2
+    out = {p.name[:-4]: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert set(out) == {"alpha", "mll", "dmll_kernel", "trace_A", "e2e_alpha", "e2e_mll", "e2e_dmll", "predict_mu",
+                        "predict_var"}
+    assert all(v.dtype == np.float64 for v in out.values())
+    assert sum(v.nbytes for v in out.values()) <= 64 << 20
+    X, y = bench.synth(n, bench.D, seed=1)
+    spec = ("SEIso", [bench.LL, bench.LSIG])
+    o = orc.mll_and_dmll(spec, X, y, bench.LNOISE, ("MeanConst", 0.0))
+    rel = lambda a, b: float(np.max(np.abs(a - b)) / np.max(np.abs(b)))
+    for m in (out["mll"], out["e2e_mll"]):
+        assert m.shape == (1,) and abs(m[0] - o["mll"]) <= 1e-10 * abs(o["mll"])
+    assert rel(out["alpha"], o["alpha"]) < 1e-10 and rel(out["e2e_alpha"], o["alpha"]) < 1e-10
+    assert rel(out["dmll_kernel"], o["dmll_kernel"]) < 1e-8 and rel(out["e2e_dmll"], o["dmll"]) < 1e-8
+    assert abs(out["trace_A"][0] - o["trA"]) <= 1e-8 * abs(o["trA"])
+    mo, vo = orc.predict_f(spec, X, o, np.random.default_rng(2).standard_normal((4096, bench.D)), ("MeanConst", 0.0))
+    assert rel(out["predict_mu"], mo) < 1e-10
+    assert np.max(np.abs(out["predict_var"] - vo)) <= 1e-10 * np.max(np.abs(vo)) + 1e-13
+
+
 @pytest.mark.parametrize("name", ["r01_final_bench_1gpu.json", "r01_final_bench_2gpu.json", "r01_final_bench_8gpu.json"])
 def test_committed_bench_lines_have_every_key(name):
     j = json.load(open(os.path.join(ROOT, "profiles", name)))
