@@ -4,10 +4,11 @@
 // Device layout (all FP64, row-major, leading dimension Npad = N rounded up to 128; the padding is
 // an identity block, so L, L^-1, logdet and every solve are unaffected):
 //   F     Npad x Npad   lower triangle: L (K_y = L L'; the reference's U = L', src/GP.jl:110).
-//                       strict-upper tiles: scratch for the triangular-inverse merges.
+//                       strict-upper tiles: scratch for the triangular-inverse merges (and Z' of gpb200_gpa_grad).
 //   G     Npad x Npad   lower tiles: K_y -> Schur complements during the factorisation ->
 //                       W = L^-1 (strictly-lower tiles) ; strictly-upper tiles: W' ;
-//                       after gpb200_grad_prepare the lower triangle holds K_y^-1.
+//                       after gpb200_grad_prepare the lower triangle holds K_y^-1,
+//                       after gpb200_gpa_grad -(P + P') of the latent-GP gradient.
 //   Dinv / DinvT  Npad x 128   clean lower / upper copies of the inverted diagonal tiles.
 //   x     N x d point-major (== Julia's d x N column-major), uploaded once (gpb200_set_data).
 // The reference keeps four N x N host matrices per GPE (R, cK.mat, chol factors, ααinvcKI;
@@ -38,6 +39,7 @@
 
 #include "../../include/gpb200.h"
 #include "gemm_nt.cuh"
+#include "gpa.cuh"
 #include "gram.cuh"
 #include "gram_fast.cuh"
 #include "kprog.cuh"
@@ -73,6 +75,12 @@ struct gpb200_handle {
     double *noise_var = nullptr, *r0 = nullptr, *r1 = nullptr, *y1 = nullptr, *alpha = nullptr, *scal = nullptr;
     double *part = nullptr, *trace_out = nullptr;
     double* tblk = nullptr;                    // Npad scratch vector (block right-hand sides of the sharded solves)
+    // latent-GP gradient (gpb200_gpa_grad): Z' diagonal tiles [Npad x 128] and [Npad/128 x Npad] per-tile partial sums
+    double *Zd = nullptr, *gpa_part = nullptr;
+    int64_t gpa_npad = 0;                      // Npad the two buffers were sized for
+    CUtensorMap mapZd{};
+    bool chol_bar_ready = false;               // G's lower triangle holds -(P + P') of the last gpb200_gpa_grad
+    cudaEvent_t ev_gpa[6] = {};                // phase boundaries of gpb200_unwhiten / gpb200_gpa_grad (timings [9..13])
     // TMA-staged SEIso kernels (gram_fast.cu): inputs stored [Npad x dxp] with an even, zero-padded dxp <= 8
     double *xp = nullptr, *xpt = nullptr;      // [Npad x dxp] and its transpose [dxp x Npad]
     int dxp = 0;
@@ -112,7 +120,7 @@ struct gpb200_handle {
     cudaStream_t st_cur = nullptr;             // stream launch_gemm / the leaf use right now (st or st_side)
     cudaEvent_t ev_la0 = nullptr, ev_la2 = nullptr;
     // stats
-    double ms[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    double ms[16] = {};
     int64_t launches = 0;
     bool own_stream = true;
     // per-launch GEMM profiling (option "profile"): event pairs + executed flops of every GEMM launch
@@ -286,7 +294,8 @@ void free_data(gpb200_handle* h) {
     free_FG(h);
     double** ptrs[] = {&h->x, &h->Dinv, &h->DinvT, &h->logd, &h->noise_var, &h->r0, &h->r1,
                        &h->y1, &h->alpha, &h->scal, &h->part, &h->trace_out, &h->xs, &h->Kst, &h->Kss,
-                       &h->pmu, &h->pvar, &h->pkdiag, &h->tblk, &h->xp, &h->xpt};
+                       &h->pmu, &h->pvar, &h->pkdiag, &h->tblk, &h->xp, &h->xpt, &h->Zd, &h->gpa_part};
+    h->gpa_npad = 0; h->chol_bar_ready = false;
     h->xmap_ok = false;
     if (h->cvD) cudaFree(h->cvD);
     if (h->cvY) cudaFree(h->cvY);
@@ -494,9 +503,10 @@ cudaError_t cholesky(gpb200_handle* h) {
     return cudaSuccess;
 }
 
-// K_y^-1 from the factor: level-parallel triangular inverse (all pairs of adjacent s x s diagonal
-// blocks merged at once, s = 128, 256, ...: 2 batched GEMM launches per level), then W'W.
-cudaError_t inverse_from_factor(gpb200_handle* h) {
+// W = L^-1 from the factor: level-parallel triangular inverse (all pairs of adjacent s x s diagonal
+// blocks merged at once, s = 128, 256, ...: 2 batched GEMM launches per level).  W' ends in G's
+// strictly-upper tiles (diagonal tiles: DinvT).
+cudaError_t inverse_merges(gpb200_handle* h) {
     const int Np = (int)h->Npad;
     cudaError_t e;
     for (long long s = TILE; s < Np; s *= 2) {
@@ -504,6 +514,14 @@ cudaError_t inverse_from_factor(gpb200_handle* h) {
         const int n2 = (int)((Np - s < s) ? Np - s : s);
         if ((e = merge_inverse(h, 0, (int)s, n2, batch)) != cudaSuccess) return e;
     }
+    return cudaSuccess;
+}
+
+// K_y^-1 from the factor: the triangular inverse, then W'W.
+cudaError_t inverse_from_factor(gpb200_handle* h) {
+    const int Np = (int)h->Npad;
+    cudaError_t e;
+    if ((e = inverse_merges(h)) != cudaSuccess) return e;
     GemmDesc g = gemm_desc_default();
     g.A = GemmOperand{bufG(h), bufDinvT(h), 0, 0};
     g.B = GemmOperand{bufG(h), bufDinvT(h), 0, 0};
@@ -929,7 +947,7 @@ cudaError_t trsm_rec(gpb200_handle* h, int Mpad, int c0, int n) {
 
 // factor whatever SPD matrix sits in the lower tiles of h->G (padding must be identity)
 int chol_inplace(gpb200_handle* h) {
-    h->factored = h->inv_ready = h->alpha_ready = false;
+    h->factored = h->inv_ready = h->alpha_ready = h->chol_bar_ready = false;
     const int init = INT_MAX;
     CK(cudaMemcpyAsync(h->info_dev, &init, sizeof(int), cudaMemcpyHostToDevice, h->st));
     CK(cholesky(h));
@@ -998,6 +1016,28 @@ int copy_own_rows(gpb200_handle* h, double* dst_host, const double* src_dev) {
 }
 int sync_all(const Locals& L) {
     for (auto* q : L) SCK(q, cudaStreamSynchronize(q->st));
+    return GPB200_OK;
+}
+
+// latent-GP entry points: single-GPU handles with a resident factor; lazily sized workspace
+int gpa_entry(gpb200_handle* h, const char* who) {
+    char buf[160];
+    if (h->nranks > 1 || h->sharded || h->grp) {
+        snprintf(buf, sizeof buf, "%s: GPA runs on single-GPU handles only (not on replicated or row-sharded multi-rank storage)", who);
+        return fail(h, GPB200_EINVAL, buf);
+    }
+    if (!h->factored) { snprintf(buf, sizeof buf, "%s: factorize first", who); return fail(h, GPB200_ESTATE, buf); }
+    CK(cudaSetDevice(h->device));
+    if (h->gpa_npad == h->Npad) return GPB200_OK;
+    if (h->Zd) cudaFree(h->Zd);
+    if (h->gpa_part) cudaFree(h->gpa_part);
+    h->Zd = h->gpa_part = nullptr; h->gpa_npad = 0;
+    CK(cudaMalloc(&h->Zd, sizeof(double) * (size_t)h->Npad * TILE));
+    CK(cudaMalloc(&h->gpa_part, sizeof(double) * (size_t)(h->Npad / TILE) * (size_t)h->Npad));
+    if (h->tma_ok && !gemm_make_tensor_map(&h->mapZd, h->Zd, h->Npad, TILE, TILE))
+        return fail(h, GPB200_ECUDA, "cuTensorMapEncodeTiled failed for the GPA diagonal-tile buffer");
+    for (auto& e : h->ev_gpa) if (!e) CK(cudaEventCreate(&e));
+    h->gpa_npad = h->Npad;
     return GPB200_OK;
 }
 
@@ -1080,6 +1120,7 @@ void gpb200_destroy(gpb200_handle* h) {
     if (h->ev3) cudaEventDestroy(h->ev3);
     if (h->ev_la0) cudaEventDestroy(h->ev_la0);
     if (h->ev_la2) cudaEventDestroy(h->ev_la2);
+    for (auto e : h->ev_gpa) if (e) cudaEventDestroy(e);
     if (h->st_side) cudaStreamDestroy(h->st_side);
     for (auto e : h->pev) cudaEventDestroy(e);
     if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
@@ -1161,7 +1202,7 @@ int gpb200_set_stream(gpb200_handle* h, void* stream) {
 
 int gpb200_get_timings(gpb200_handle* h, double* ms, int32_t n) {
     if (!h || !ms) return GPB200_EINVAL;
-    for (int i = 0; i < n && i < 12; ++i) ms[i] = h->ms[i];
+    for (int i = 0; i < n && i < 16; ++i) ms[i] = h->ms[i];
     return GPB200_OK;
 }
 
@@ -1290,7 +1331,7 @@ int gpb200_factorize(gpb200_handle* h, const double* theta, const double* log_no
     for (int i = 0; i < h->prog.n_theta; ++i)
         if (!isfinite(theta[i])) return fail(h, GPB200_EINVAL, "factorize: non-finite hyper-parameter");
     CK(cudaSetDevice(h->device));
-    h->factored = h->inv_ready = h->alpha_ready = false; h->g_sym = false; h->cv_m_ok = false;
+    h->factored = h->inv_ready = h->alpha_ready = false; h->g_sym = false; h->cv_m_ok = false; h->chol_bar_ready = false;
     std::vector<double> nv((size_t)n_noise);
     for (int64_t i = 0; i < n_noise; ++i) {
         if (!isfinite(log_noise[i])) return fail(h, GPB200_EINVAL, "factorize: non-finite logNoise");
@@ -1442,7 +1483,7 @@ int gpb200_grad_prepare(gpb200_handle* h) {
     if (!h) return GPB200_EINVAL;
     if (!h->factored) return fail(h, GPB200_ESTATE, "grad_prepare: factorize first");
     if (h->inv_ready) return GPB200_OK;
-    h->g_sym = false; h->cv_m_ok = false;
+    h->g_sym = false; h->cv_m_ok = false; h->chol_bar_ready = false;
     CK(cudaSetDevice(h->device));
     CK(cudaEventRecord(h->ev0, h->st));
     if (h->sharded) {
@@ -1508,6 +1549,91 @@ int gpb200_grad_kernel(gpb200_handle* h, const double* alpha, double* dmll_kerne
     h->ms[4] = ev_ms(h->ev0, h->ev1);
     if (dmll_kernel) for (int p = 0; p < np; ++p) dmll_kernel[p] = out[p];
     if (trA) *trA = out[np];
+    return GPB200_OK;
+}
+
+int gpb200_unwhiten(gpb200_handle* h, const double* v, double* f) {
+    if (!h || !v || !f) return GPB200_EINVAL;
+    { int rc = gpa_entry(h, "unwhiten"); if (rc) return rc; }
+    int rc = upload_padded(h, h->r0, v);
+    if (rc) return rc;
+    CK(cudaEventRecord(h->ev_gpa[0], h->st));
+    CK(gpa_trmv(h->F, h->ld, h->Npad, false, h->r0, h->gpa_part, h->r1, h->st, &h->launches));
+    CK(cudaEventRecord(h->ev_gpa[1], h->st));
+    CK(cudaMemcpyAsync(f, h->r1, sizeof(double) * h->N, cudaMemcpyDeviceToHost, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    h->ms[9] = ev_ms(h->ev_gpa[0], h->ev_gpa[1]);
+    return GPB200_OK;
+}
+
+// Closed-form reverse-mode Cholesky (DESIGN.md section 9.4).  With W = L^-1, w = L' g and Phi(X) = tril(X) with the
+// diagonal halved, the reference's chol_unblocked_rev! on tril(g v') contracted with dK (GPA.jl:164-173) equals
+// 1/2 sum_ij (P + P')_ij dK_ij with P = W' Z, Z = Phi(w v') W.  Schedule (launches only, all on the stream):
+//   w = L' g ; the inverse merges (W' in G's upper tiles) ; the row scan (Z' into F's upper tiles + Zd) ;
+//   G_lower = -(W' Z + Z' W) as two NT GEMMs over k >= row ; the kernel-gradient trace with alpha = 0 (A = -G).
+int gpb200_gpa_grad(gpb200_handle* h, const double* v, const double* dl_df, double* dll_v, double* dll_kernel) {
+    if (!h || !v || !dl_df) return GPB200_EINVAL;
+    { int rc = gpa_entry(h, "gpa_grad"); if (rc) return rc; }
+    // G's lower triangle is about to be overwritten: K^-1, its symmetric mirror and the CV products are gone
+    h->inv_ready = h->g_sym = h->cv_m_ok = h->chol_bar_ready = false;
+    int rc = upload_padded(h, h->r0, v);
+    if (!rc) rc = upload_padded(h, h->r1, dl_df);
+    if (rc) return rc;
+    const int Np = (int)h->Npad;
+    cudaEvent_t* ev = h->ev_gpa;
+    CK(cudaEventRecord(ev[0], h->st));
+    CK(gpa_trmv(h->F, h->ld, h->Npad, true, h->r1, h->gpa_part, h->y1, h->st, &h->launches));
+    CK(cudaEventRecord(ev[1], h->st));
+    CK(inverse_merges(h));
+    CK(cudaEventRecord(ev[2], h->st));
+    CK(gpa_row_scan(h->G, h->ld, h->DinvT, h->r0, h->y1, h->Npad, h->gpa_part, h->F, h->Zd, h->st, &h->launches));
+    CK(cudaEventRecord(ev[3], h->st));
+    const GemmBuf bZd{h->tma_ok ? &h->mapZd : nullptr, h->Zd, TILE};
+    for (int pass = 0; pass < 2; ++pass) {                 // P = W'Z (A = W', B = Z'), then P' (A = Z', B = W')
+        const GemmOperand Wt{bufG(h), bufDinvT(h), 0, 0}, Zt{bufF(h), bZd, 0, 0};
+        GemmDesc g = gemm_desc_default();
+        g.A = pass == 0 ? Wt : Zt;
+        g.B = pass == 0 ? Zt : Wt;
+        g.C = h->G; g.ldc = h->ld; g.c_row0 = 0; g.c_col0 = 0;
+        g.M = Np; g.N = Np; g.K = Np;
+        g.alpha = -1.0; g.beta = pass == 0 ? 0.0 : 1.0;
+        g.flags = GEMM_LOWER_ONLY | GEMM_KLO_M;
+        CK(launch_gemm(h, g));
+    }
+    CK(cudaEventRecord(ev[4], h->st));
+    CK(cudaMemsetAsync(h->alpha, 0, sizeof(double) * h->Npad, h->st));
+    h->alpha_ready = false;
+    h->launches += 2;
+    CK(launch_trace(h, 1, 0, 1));
+    CK(cudaEventRecord(ev[5], h->st));
+    const int np = h->prog.n_theta;
+    std::vector<double> out((size_t)np + 1);
+    CK(cudaMemcpyAsync(out.data(), h->trace_out, sizeof(double) * (np + 1), cudaMemcpyDeviceToHost, h->st));
+    if (dll_v) CK(cudaMemcpyAsync(dll_v, h->y1, sizeof(double) * h->N, cudaMemcpyDeviceToHost, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    profile_collect(h);
+    h->ms[10] = ev_ms(ev[0], ev[1]);
+    h->ms[11] = ev_ms(ev[1], ev[2]);
+    h->ms[12] = ev_ms(ev[2], ev[3]);
+    h->ms[13] = ev_ms(ev[3], ev[4]);
+    h->ms[4] = ev_ms(ev[4], ev[5]);
+    if (dll_kernel) for (int p = 0; p < np; ++p) dll_kernel[p] = out[p];
+    h->chol_bar_ready = true;
+    return GPB200_OK;
+}
+
+int gpb200_get_chol_bar(gpb200_handle* h, double* out) {
+    if (!h || !out) return GPB200_EINVAL;
+    if (!h->chol_bar_ready) return fail(h, GPB200_ESTATE, "get_chol_bar: gpa_grad first");
+    CK(cudaSetDevice(h->device));
+    const int64_t N = h->N;
+    CK(cudaMemcpy2DAsync(out, sizeof(double) * N, h->G, sizeof(double) * h->ld, sizeof(double) * N, N,
+                         cudaMemcpyDeviceToHost, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    for (int64_t i = 0; i < N; ++i) {                      // G holds -(P + P') in its lower triangle
+        for (int64_t j = 0; j < i; ++j) out[j * N + i] = out[i * N + j] = -out[i * N + j];
+        out[i * N + i] = -out[i * N + i];
+    }
     return GPB200_OK;
 }
 
@@ -1701,7 +1827,7 @@ int gpb200_append(gpb200_handle* h, int64_t k, const double* xnew, int64_t ldx) 
                      gemm_make_tensor_map_plain(&h->mapXT, h->xpt, h->dxp, Nnew, Np, h->dxp, TILE);
     }
     h->N = Nnew;
-    h->inv_ready = h->alpha_ready = false; h->g_sym = false; h->cv_m_ok = false;
+    h->inv_ready = h->alpha_ready = false; h->g_sym = false; h->cv_m_ok = false; h->chol_bar_ready = false;
     const int init = INT_MAX;
     CK(cudaMemcpyAsync(h->info_dev, &init, sizeof(int), cudaMemcpyHostToDevice, h->st));
     ++h->launches;

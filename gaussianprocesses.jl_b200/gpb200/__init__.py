@@ -7,4 +7,6 @@ from .kernels import (Kernel, SEIso, SEArd, SE, Mat12Iso, Mat32Iso, Mat52Iso, Ma
 from .means import Mean, MeanZero, MeanConst, MeanLin
 from .gpe import GPE, GP, ElasticGPE
 from .sparse import FITC, DTC, SoR
+from .likelihoods import Likelihood, BernLik, BinLik, ExpLik, GaussLik, PoisLik, StuTLik
+from .gpa import GPA
 from . import dist

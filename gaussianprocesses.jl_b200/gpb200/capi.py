@@ -36,6 +36,9 @@ _SIGNATURES = {
     "gpb200_mll": (C.c_int, [_H, _dp, _dp, _dp]),
     "gpb200_grad_prepare": (C.c_int, [_H]),
     "gpb200_grad_kernel": (C.c_int, [_H, _dp, _dp, _dp]),
+    "gpb200_unwhiten": (C.c_int, [_H, _dp, _dp]),
+    "gpb200_gpa_grad": (C.c_int, [_H, _dp, _dp, _dp, _dp]),
+    "gpb200_get_chol_bar": (C.c_int, [_H, _dp]),
     "gpb200_predict": (C.c_int, [_H, C.c_int64, _dp, C.c_int64, _dp, _dp, _dp, _dp]),
     "gpb200_rand": (C.c_int, [_H, C.c_int64, _dp, C.c_int64, _dp, C.c_int64, _dp, C.c_double, _dp, _dp]),
     "gpb200_append": (C.c_int, [_H, C.c_int64, _dp, C.c_int64]),
@@ -206,6 +209,32 @@ class Engine:
         self._check(self._lib.gpb200_grad_kernel(self._h, ap, _as_dp(g), C.byref(tr)), "grad_kernel")
         return g[:self.n_theta].copy(), tr.value
 
+    def unwhiten(self, v):
+        """f = L v on the resident factor (GPA.jl:106)."""
+        v = np.ascontiguousarray(v, dtype=np.float64)
+        if v.shape != (self.N,):
+            raise ValueError("unwhiten: v must have length N")
+        f = np.empty(self.N)
+        self._check(self._lib.gpb200_unwhiten(self._h, _as_dp(v), _as_dp(f)), "unwhiten")
+        return f
+
+    def gpa_grad(self, v, dl_df):
+        """(L' dl_df, dll_kern) of the latent GP (GPA.jl:183-228); K^-1 and the resident alpha are gone afterwards."""
+        v = np.ascontiguousarray(v, dtype=np.float64)
+        g = np.ascontiguousarray(dl_df, dtype=np.float64)
+        if v.shape != (self.N,) or g.shape != (self.N,):
+            raise ValueError("gpa_grad: v and dl_df must have length N")
+        dv = np.empty(self.N)
+        dk = np.empty(max(self.n_theta, 1))
+        self._check(self._lib.gpb200_gpa_grad(self._h, _as_dp(v), _as_dp(g), _as_dp(dv), _as_dp(dk)), "gpa_grad")
+        return dv, dk[:self.n_theta].copy()
+
+    def chol_bar(self):
+        """debug: the symmetric P + P' of the last gpa_grad"""
+        out = np.empty((self.N, self.N))
+        self._check(self._lib.gpb200_get_chol_bar(self._h, _as_dp(out)), "get_chol_bar")
+        return out
+
     def predict(self, xs_pm, alpha=None, want_var=True, full_cov=False):
         xs_pm = np.ascontiguousarray(xs_pm, dtype=np.float64)
         M, d = xs_pm.shape
@@ -291,10 +320,11 @@ class Engine:
         return np.tril(K)
 
     def timings(self):
-        ms = np.zeros(12)
-        self._check(self._lib.gpb200_get_timings(self._h, _as_dp(ms), 12), "get_timings")
+        ms = np.zeros(16)
+        self._check(self._lib.gpb200_get_timings(self._h, _as_dp(ms), 16), "get_timings")
         return dict(gram=ms[0], cholesky=ms[1], solve_mll=ms[2], inverse=ms[3], trace=ms[4], predict=ms[5],
-                    gemm_launches=ms[6], gemm_ms=ms[7], gemm_flops=ms[8])
+                    gemm_launches=ms[6], gemm_ms=ms[7], gemm_flops=ms[8], gpa_unwhiten=ms[9], gpa_trmv_t=ms[10],
+                    gpa_merges=ms[11], gpa_scan=ms[12], gpa_gemms=ms[13])
 
     def set_stream(self, cuda_stream):
         """Run on the caller's CUDA stream (int handle, e.g. torch.cuda.current_stream().cuda_stream); 0/None = private."""
@@ -508,6 +538,12 @@ class LocalGroupEngine:
 
     def predict(self, *a, **k):
         return self.lead.predict(*a, **k)
+
+    def unwhiten(self, *a, **k):
+        return self.lead.unwhiten(*a, **k)
+
+    def gpa_grad(self, *a, **k):
+        return self.lead.gpa_grad(*a, **k)
 
     def rand(self, *a, **k):
         return self.lead.rand(*a, **k)

@@ -399,6 +399,12 @@ class GPE:
 
 
 def GP(x, y, mean, kernel, logNoise=-2.0, **kw):                   # GPE.jl:119
+    """GP(x, y, mean, kernel, logNoise) builds a GPE; GP(x, y, mean, kernel, lik) with a Likelihood builds a GPA
+    (GPA.jl:93-94)."""
+    from .likelihoods import Likelihood
+    if isinstance(logNoise, Likelihood):
+        from .gpa import GPA
+        return GPA(x, y, mean, kernel, logNoise, **kw)
     return GPE(x, y, mean, kernel, logNoise, **kw)
 
 

@@ -346,6 +346,135 @@ function Random.rand!(gp::GPE{X,Y,M,K,CS,D,P}, x::AbstractMatrix, A::DenseMatrix
 end
 
 # =====================================================================================================
+# Latent-variable GP (src/GPA.jl) on the device.  The reference's GPA hard-codes cK::PDMat{Float64,Matrix{Float64}}, so
+# the binding is a GPBase of its own with GPA's fields and methods; mcmc / ess / optimize! drive it unchanged.  The
+# device keeps the factor: update_cK! (GPA.jl:111-114), unwhiten (f = L v) and the gradient's reverse-mode Cholesky
+# contracted with dK/dθ (gpb200_gpa_grad) never bring an N x N matrix to the host.
+import GaussianProcesses: GPBase, Likelihood, log_dens, dlog_dens_df, dlog_dens_dθ, predict_obs, predict_y,
+                          initialise_target!, update_dtarget!, update_target_and_dtarget!, set_params!, grad_stack,
+                          prior_logpdf, prior_gradlogpdf, get_params_kwargs
+
+mutable struct B200GPA{L<:Likelihood} <: GPBase
+    x::Matrix{Float64}
+    y::AbstractVector
+    mean::Mean
+    kernel::Kernel
+    lik::L
+    dim::Int
+    nobs::Int
+    v::Vector{Float64}
+    μ::Vector{Float64}
+    cK::B200PDMat
+    ll::Float64
+    dll::Vector{Float64}
+    target::Float64
+    dtarget::Vector{Float64}
+    function B200GPA(x::AbstractMatrix, y::AbstractVector, mean::Mean, kernel::Kernel, lik::L; device::Int = 0) where {L<:Likelihood}
+        dim, nobs = size(x)
+        length(y) == nobs || throw(ArgumentError("Input and output observations must have consistent dimensions."))
+        gp = new{L}(Matrix{Float64}(x), y, mean, kernel, lik, dim, nobs, zeros(nobs), zeros(nobs), B200PDMat(device, nobs),
+                    NaN, Float64[], NaN, Float64[])
+        return initialise_target!(gp)
+    end
+end
+
+function b200_unwhiten(cK::B200PDMat, v::Vector{Float64})                      # unwhiten(cK, v), GPA.jl:106
+    f = Vector{Float64}(undef, cK.n)
+    check(cK, ccall((:gpb200_unwhiten, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}), cK.handle, v, f), "unwhiten")
+    return f
+end
+
+function gpa_set_target!(gp::B200GPA)                                           # GPA.jl:247-248, 263-264
+    gp.μ = mean(gp.mean, gp.x)
+    gp.ll = sum(log_dens(gp.lik, b200_unwhiten(gp.cK, gp.v) + gp.μ, gp.y))
+    gp.target = gp.ll - (sum(abs2, gp.v) + log(2π) * gp.nobs) / 2 +
+        prior_logpdf(gp.lik) + prior_logpdf(gp.mean) + prior_logpdf(gp.kernel)
+    return gp
+end
+
+function initialise_target!(gp::B200GPA)                                        # GPA.jl:101-109: Σ + 1e-6 I
+    b200_update!(gp.cK, gp.x, gp.kernel, [0.5 * log(1e-6)])
+    return gpa_set_target!(gp)
+end
+
+function update_target!(gp::B200GPA; process::Bool=true, lik::Bool=true, domean::Bool=true, kern::Bool=true)   # GPA.jl:261-266
+    kern && b200_update!(gp.cK, gp.x, gp.kernel, [-20.0])                   # update_cK!, GPA.jl:111-114
+    return gpa_set_target!(gp)
+end
+
+function update_dtarget!(gp::B200GPA; process::Bool=true, lik::Bool=true, domean::Bool=true, kern::Bool=true)  # GPA.jl:183-228, 268-272
+    f = b200_unwhiten(gp.cK, gp.v) + gp.μ
+    dl_df = Vector{Float64}(dlog_dens_df(gp.lik, f, gp.y))
+    dv = Vector{Float64}(undef, gp.nobs); g = Vector{Float64}(undef, max(gp.cK.ntheta, 1))
+    if process || kern                                                          # L' dl_df and dll_kern! in one device call
+        check(gp.cK, ccall((:gpb200_gpa_grad, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                           gp.cK.handle, gp.v, dl_df, dv, g), "gpa_grad")
+    end
+    dll = Float64[]
+    process && append!(dll, dv)
+    lik && num_params(gp.lik) > 0 && append!(dll, vec(sum(dlog_dens_dθ(gp.lik, f, gp.y), dims=1)))
+    domean && num_params(gp.mean) > 0 && append!(dll, grad_stack(gp.mean, gp.x)' * dl_df)
+    kern && append!(dll, g[gp.cK.exposed])
+    gp.dll = dll
+    gp.dtarget = dll + prior_gradlogpdf(gp; process=process, lik=lik, domean=domean, kern=kern)
+    return gp
+end
+
+function update_target_and_dtarget!(gp::B200GPA; kwargs...)                      # GPA.jl:283-291
+    update_target!(gp; kwargs...)
+    return update_dtarget!(gp; kwargs...)
+end
+update_target_and_dtarget!(gp::B200GPA, ::AbstractGradientPrecompute; kwargs...) = update_target_and_dtarget!(gp; kwargs...)
+init_precompute(gp::B200GPA) = B200Precompute()
+get_params_kwargs(::B200GPA; kwargs...) = delete!(Dict(kwargs), :noise)          # src/optimize.jl:2
+
+function prior_gradlogpdf(gp::B200GPA; process::Bool=true, lik::Bool=true, domean::Bool=true, kern::Bool=true)  # GPA.jl:383-399
+    grad = process ? -gp.v : Float64[]
+    lik && append!(grad, prior_gradlogpdf(gp.lik))
+    domean && append!(grad, prior_gradlogpdf(gp.mean))
+    kern && append!(grad, prior_gradlogpdf(gp.kernel))
+    return grad
+end
+
+function get_params(gp::B200GPA; lik::Bool=true, domean::Bool=true, kern::Bool=true)   # GPA.jl:336-349
+    params = copy(gp.v)
+    lik && num_params(gp.lik) > 0 && append!(params, get_params(gp.lik))
+    domean && num_params(gp.mean) > 0 && append!(params, get_params(gp.mean))
+    kern && append!(params, get_params(gp.kernel))
+    return params
+end
+num_params(gp::B200GPA; lik::Bool=true, domean::Bool=true, kern::Bool=true) =      # GPA.jl:351-357
+    gp.nobs + (lik ? num_params(gp.lik) : 0) + (domean ? num_params(gp.mean) : 0) + (kern ? num_params(gp.kernel) : 0)
+
+function set_params!(gp::B200GPA, hyp::AbstractVector; process::Bool=true, lik::Bool=true, domean::Bool=true, kern::Bool=true)  # GPA.jl:359-381
+    nl, nm, nk = num_params(gp.lik), num_params(gp.mean), num_params(gp.kernel)
+    i = 1
+    if process
+        gp.v = hyp[1:gp.nobs]; i += gp.nobs
+    end
+    if lik && nl > 0
+        set_params!(gp.lik, hyp[i:i+nl-1]); i += nl
+    end
+    if domean && nm > 0
+        set_params!(gp.mean, hyp[i:i+nm-1]); i += nm
+    end
+    kern && set_params!(gp.kernel, hyp[i:i+nk-1])
+end
+
+function predict_f(gp::B200GPA, x::AbstractMatrix; full_cov::Bool=false)          # predict_full, GPA.jl:294
+    size(x, 1) == gp.dim || throw(ArgumentError("Gaussian Process object and input observations do not have consistent dimensions"))
+    alpha = gp.cK \ b200_unwhiten(gp.cK, gp.v)
+    mu, s = predict_raw(gp.cK, x, alpha, full_cov)
+    mu = mu .+ mean(gp.mean, Matrix{Float64}(x))
+    return full_cov ? (mu, s) : (mu, max.(s, 0.0))                                   # src/GP.jl:75
+end
+
+function predict_y(gp::B200GPA, x::AbstractMatrix; full_cov::Bool=false)          # GPA.jl:303-306
+    μ, σ2 = predict_f(gp, x; full_cov=full_cov)
+    return predict_obs(gp.lik, μ, σ2)
+end
+
+# =====================================================================================================
 # Sparse strategies on the device: FITC / DTC / SoR (src/sparse/*.jl) -> gpb200_fitc_* (one streaming engine)
 #     gp = GPE(x, y, mean, kernel, logNoise, B200Sparse(Xu, :FITC))
 # =====================================================================================================
@@ -446,6 +575,6 @@ function predict_f(gp::GPE{X,Y,M,K,CS,D,P}, x::AbstractMatrix; full_cov::Bool=fa
     return mu .+ mean(gp.mean, Xs), max.(var, 0.0)
 end
 
-export B200Covariance, B200Sparse, B200ElasticGPE
+export B200Covariance, B200Sparse, B200ElasticGPE, B200GPA
 
 end # module

@@ -114,6 +114,22 @@ int  gpb200_grad_prepare(gpb200_handle* h);
  * `alpha` may be NULL to use the alpha left resident by gpb200_mll.                          */
 int  gpb200_grad_kernel(gpb200_handle* h, const double* alpha, double* dmll_kernel, double* trA);
 
+/* ---- latent-variable GP (src/GPA.jl; single-GPU handles, after gpb200_factorize) -------------------------------------
+ * GPA whitens the latent values, f = L v + mu with K = L L' (the shim factorises with logNoise = -20, GPA.jl:111-114).
+ * Multi-rank handles (replicated or row-sharded) return GPB200_EINVAL.                                                 */
+/* unwhiten(cK, v) (GPA.jl:106,125,159): f = L v, both length N on host                                                 */
+int  gpb200_unwhiten(gpb200_handle* h, const double* v, double* f);
+/* update_dll! (GPA.jl:183-228), process and kernel blocks: dll_v[N] = L' dl_df (may be NULL; GPA.jl:200) and
+ * dll_kernel[n_theta] = dll_kern! (GPA.jl:164-173: chol_unblocked_rev! on tril(dl_df v'), diagonal doubled, dmll_kern!),
+ * computed in closed form: 1/2 sum_ij (P + P')_ij dK_ij/dtheta_p with P = W' Phi(w v') W, W = L^-1, w = L' dl_df,
+ * Phi = lower triangle with the diagonal halved.  G no longer holds K^-1 afterwards: gpb200_grad_kernel, the
+ * cross-validation calls and gpb200_get_inverse(_diag) return GPB200_ESTATE until gpb200_grad_prepare runs again, and
+ * the resident alpha is cleared (pass alpha explicitly to gpb200_predict).  solve, logdet, predict and unwhiten keep
+ * working on the unchanged factor.                                                                                     */
+int  gpb200_gpa_grad(gpb200_handle* h, const double* v, const double* dl_df, double* dll_v, double* dll_kernel);
+/* debug: the N x N symmetric P + P' of the last gpb200_gpa_grad (row-major)                                           */
+int  gpb200_get_chol_bar(gpb200_handle* h, double* out);
+
 /* ---- predictMVN / predict_f (src/GP.jl:25-79) ---------------------------------------------
  * xs: d x M column-major test inputs (leading dim ldxs).  mu_minus_mean[M] = K*' alpha;
  * var[M] (may be NULL) = k** - |L^-1 k*|^2, NOT clamped (the shim applies max(.,0) as
@@ -157,7 +173,9 @@ int  gpb200_get_inverse_diag(gpb200_handle* h, double* diag);
  * [0] gram  [1] cholesky  [2] solve+mll  [3] inverse (trtri+lauum)  [4] trace  [5] predict
  * with option "profile"=1, accumulated since the option was set:
  * [6] number of DMMA GEMM launches  [7] sum of their device durations (ms, CUDA events around
- * every launch)  [8] FP64 flops those launches executed (tile-granular)                       */
+ * every launch)  [8] FP64 flops those launches executed (tile-granular)
+ * of the last gpb200_unwhiten / gpb200_gpa_grad: [9] L v  [10] L' g  [11] inverse merges  [12] row scan
+ * [13] the two GEMMs of P + P'  (the trace of gpb200_gpa_grad goes to [4]); up to n = 16 values    */
 int  gpb200_get_timings(gpb200_handle* h, double* ms, int32_t n);
 /* number of kernel launches issued by this handle since creation */
 int64_t gpb200_launch_count(gpb200_handle* h);
